@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              # this repo (CUDA kernels), through the node API
     python bench.py --impl reference --gpus N --steps K ...    # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                     # also write what the last timed step returned (.npy)
 
 What is measured (`config.workload`): `requests_per_gpu` independent SDXL inpaint requests of shape [1,4,128,128]
 (BASELINE configs[1]'s latent) batched per GPU, each running the reference schedule: karras-20 sigmas x N=5 think
@@ -388,7 +389,7 @@ class NodeWorkload:
         if self.spec.sampler != "euler":           # other samplers evaluate the wrapper at sigmas of their own
             eng = self.N.LAST_ENGINE["engine"]
             self.substeps, self.guider_calls = eng.substeps_done, eng.model_calls
-        self.last_out = out["samples"]
+        self.last_out = out                        # the LATENT dict the caller receives
         return wall, e0.elapsed_time(e1)
 
     def warm(self, n=8):
@@ -433,6 +434,34 @@ class NodeWorkload:
                 "graphs": job.captures if job is not None else None}
 
 
+class OutputDump:
+    """--dump-outputs: what the timed path handed back in its last step, so that two builds run with the same arguments
+    can be compared output for output.  Every array of each call's LATENT dict is stacked over the step's calls and
+    written as DIR/<key>.npy (float32).  When the whole step exceeds `budget` bytes, each call contributes the same fixed
+    sample of flat element indices: the first n of torch.randperm(numel) under a generator seeded with 0, sorted."""
+
+    def __init__(self, calls: int, budget: int = 60 * 10 ** 6):     # under 64 MB with the .npy headers
+        self.calls, self.budget, self.rows, self.index = calls, budget, {}, {}
+
+    def add(self, latent):
+        arrays = {k: v for k, v in latent.items() if isinstance(v, torch.Tensor)}
+        total = 4 * self.calls * sum(v.numel() for v in arrays.values())
+        for key, v in arrays.items():
+            v = v.detach().float().cpu()
+            if total > self.budget:
+                if key not in self.index:
+                    n = v.numel() * self.budget // total
+                    self.index[key] = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+                v = v.reshape(-1)[self.index[key]]
+            self.rows.setdefault(key, []).append(v.clone())
+
+    def write(self, out_dir: str):
+        import numpy as np
+        os.makedirs(out_dir, exist_ok=True)
+        for key, rows in self.rows.items():
+            np.save(os.path.join(out_dir, key + ".npy"), torch.stack(rows).numpy())
+
+
 class DirectGuider:
     """The object the engine sees from ComfyUI's patched CFGGuider, without ComfyUI: cond / uncond evaluations of
     the same synthetic network, handed over as a CfgPair (both CFG combines happen in the update kernel)."""
@@ -470,21 +499,25 @@ def run_b200(args):
     spec_main = Spec("sdxl_batch", R, SHAPE)
     other_rng = "philox" if args.rng == "torch" else "torch"
 
-    def measure(spec, rng, steps, warm_steps, jobs, seed=rank, tag=None):
-        """steps x jobs node calls: device time of the sampler loops (sum, max over ranks) and wall time."""
+    def measure(spec, rng, steps, warm_steps, jobs, seed=rank, tag=None, dump=None):
+        """steps x jobs node calls: device time of the sampler loops (sum, max over ranks) and wall time.  `dump`: an
+        OutputDump that receives what each call of the last step returned."""
         wl = NodeWorkload(spec, dev, rng, seed=seed)
         wl.net.coef = tuple(weights.tolist())
         wl.warm()
         for _ in range(warm_steps * jobs):
             wl.call()
+        wl.seed = 1000 * (seed + 1) + 10 ** 6     # timed calls draw the same seeds however many calls warming took
         group.barrier()
         if tag == "main":
             clocks.mark("t0")
         span_ms, wall_s = 0.0, 0.0
-        for _ in range(steps * jobs):
+        for i in range(steps * jobs):
             w_, s_ = wl.call()
             wall_s += w_
             span_ms += s_
+            if dump is not None and i >= (steps - 1) * jobs:
+                dump.add(wl.last_out)             # outside call(): neither clock sees it
         group.barrier()
         if tag == "main":
             clocks.mark("t1")
@@ -498,7 +531,10 @@ def run_b200(args):
         return rec, wl
 
     # ---- main line: the node API at the shipped default -------------------------------------------------------
-    main, wl_main = measure(spec_main, args.rng, K, W, J, tag="main")
+    dump = OutputDump(J) if args.dump_outputs and rank == 0 else None
+    main, wl_main = measure(spec_main, args.rng, K, W, J, tag="main", dump=dump)
+    if dump is not None:
+        dump.write(args.dump_outputs)
     noise_ms, cpu_noise_ms, noise_where = wl_main.prepare_noise_ms()
     on_device = noise_where.startswith("device")
     wl_main.h2d = wl_main.h2d - (wl_main.latent["samples"].numel() * 4 if on_device else 0)   # no noise image to upload
@@ -991,7 +1027,12 @@ def main():
                     help="InnerThreshold of the frame-sharded record that runs with the early stopper on")
     ap.add_argument("--mask", default="random", choices=["random", "blob"],
                     help="random 50%% per site (SURVEY 8d, default) | one centred hole of about the same area")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the main line's last timed step returned as DIR/<key>.npy (float32, <= 64 MB in "
+                         "all; a fixed seeded sample when larger); rank 0 only, b200 impl only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global MASK_KIND
     MASK_KIND = args.mask
     if args.impl == "reference":

@@ -1,7 +1,7 @@
 """Generate golden vectors from the REAL reference engine (run in the build container only).
 
     python tests/golden/make_golden.py            # writes every fixture under tests/golden/
-    python tests/golden/make_golden.py --engine   # or one family: --engine | --api | --earlystop | --av
+    python tests/golden/make_golden.py --engine   # or one family: --engine | --api | --node-units | --ref-port | --earlystop | --av
 
 The reference (`/root/reference/src/LanPaint/lanpaint.py`, imported unmodified)
 is driven with stand-in denoisers that follow its own test doubles' protocol
@@ -30,6 +30,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, "/root/reference")
 
 from oracle import langevin_oracle as O  # noqa: E402
@@ -149,31 +150,8 @@ RESHAPE_CASES = {
 
 def dump_node_api():
     import importlib
-    import types
-
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        for k, v in attrs.items():
-            setattr(m, k, v)
-        sys.modules[name] = m
-        return m
-
-    comfy = stub("comfy")
-    comfy.__path__ = []
-    def _repeat(t, n):  # comfy.utils.repeat_to_batch_size semantics
-        if t.shape[0] >= n:
-            return t[:n]
-        reps = (n + t.shape[0] - 1) // t.shape[0]
-        return t.repeat((reps,) + (1,) * (t.ndim - 1))[:n]
-
-    comfy.utils = stub("comfy.utils", repeat_to_batch_size=_repeat)
-    comfy.samplers = stub("comfy.samplers", KSAMPLER=type("KSAMPLER", (), {}),
-                          KSampler=type("KSampler", (), {"SCHEDULERS": ["<SCHEDULERS>"]}))
-    comfy.model_base = stub("comfy.model_base", ModelType=types.SimpleNamespace(FLUX="FLUX", FLOW="FLOW"),
-                            WAN22=type("WAN22", (), {}))
-    stub("nodes")
-    stub("latent_preview")
-    stub("comfyui_version", __version__="0.6.0")
+    from _node_unit_cases import install_comfy_stubs
+    install_comfy_stubs()
     ref = importlib.import_module("src.LanPaint.nodes")
     api = {}
     for name in ("LanPaint_KSampler", "LanPaint_KSamplerAdvanced", "LanPaint_SamplerCustom",
@@ -202,6 +180,35 @@ def dump_node_api():
               "comfyui_version", "src.LanPaint.nodes"):
         sys.modules.pop(n, None)
     print("node_api.json written")
+
+
+def dump_ref_port():
+    """The reference engine's outputs on tests/test_oracle_ref.py's cases (same inputs, same noise tape)."""
+    import pytest
+    import test_oracle_ref as T
+    arrays = {}
+    for flow, n, batch in T.CASES:
+        args, _, draws = T.port_case(flow, n, batch)
+        with pytest.MonkeyPatch.context() as mp:
+            out, x = T.run_reference(RefEngine, flow, n, args, draws, mp)
+        arrays[f"{int(flow)}_{n}_{batch}_out"], arrays[f"{int(flow)}_{n}_{batch}_x"] = out.numpy(), x.numpy()
+    np.savez_compressed(os.path.join(HERE, "aux_ref_port_cases.npz"), **arrays)
+    print("aux_ref_port_cases.npz written")
+
+
+def dump_node_units():
+    """The reference node module's answers to the unit-level calls of tests/_node_unit_cases.py."""
+    import importlib
+    import _node_unit_cases
+    _node_unit_cases.install_comfy_stubs()
+    ref = importlib.import_module("src.LanPaint.nodes")
+    with open(os.path.join(HERE, "node_unit_answers.json"), "w") as f:
+        json.dump(_node_unit_cases.run(ref), f, separators=(",", ":"))
+        f.write("\n")
+    for n in ("comfy", "comfy.utils", "comfy.samplers", "comfy.model_base", "nodes", "latent_preview",
+              "comfyui_version", "src.LanPaint.nodes"):
+        sys.modules.pop(n, None)
+    print("node_unit_answers.json written")
 
 
 
@@ -315,9 +322,11 @@ def dump_av():
 
 if __name__ == "__main__":
     # python tests/golden/make_golden.py            -> everything
-    # python tests/golden/make_golden.py --engine   -> only the engine cases (likewise --api, --earlystop, --av)
+    # python tests/golden/make_golden.py --engine   -> only the engine cases (likewise --api, --node-units, --ref-port,
+    #                                                   --earlystop, --av)
     picked = [a for a in sys.argv[1:] if a.startswith("--")]
-    todo = {"--engine": main, "--api": dump_node_api, "--earlystop": dump_earlystop, "--av": dump_av}
+    todo = {"--engine": main, "--api": dump_node_api, "--node-units": dump_node_units, "--ref-port": dump_ref_port,
+            "--earlystop": dump_earlystop, "--av": dump_av}
     for flag, fn in todo.items():
         if not picked or flag in picked:
             fn()

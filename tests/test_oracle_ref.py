@@ -1,17 +1,22 @@
 """oracle/_ref (the reference's own engine, compiled to bytecode by oracle/build_ref.py) against the oracle port:
-the thing bench.py times as `cpu_baseline.kind == "reference"` is the code the port restates, bit for bit."""
+the thing bench.py times as `cpu_baseline.kind == "reference"` is the code the port restates, bit for bit.  The
+reference engine's outputs for the same cases are also stored (tests/golden/aux_ref_port_cases.npz, written by
+tests/golden/make_golden.py --ref-port), so the port is held to them where oracle/_ref is not built."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
+from conftest import GOLDEN_DIR
 from oracle import build_ref
 from oracle import langevin_oracle as O
 
+CASES = [(False, 5, 1), (False, 3, 2), (True, 4, 1)]
 
-@pytest.mark.parametrize("flow,n,batch", [(False, 5, 1), (False, 3, 2), (True, 4, 1)])
-def test_reference_bytecode_equals_the_port(flow, n, batch, monkeypatch):
-    Ref = build_ref.load()
-    if Ref is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference: `make -C oracle`)")
+
+def port_case(flow, n, batch):
+    """-> (engine arguments, the port's (out, x), its noise tape) of one case."""
     g = torch.Generator().manual_seed(3)
     shape = (batch, 4, 16, 16)
     x, y, noise = (torch.randn(shape, generator=g) for _ in range(3))
@@ -19,16 +24,35 @@ def test_reference_bytecode_equals_the_port(flow, n, batch, monkeypatch):
     sigma = torch.full((batch,), 0.6 if flow else 2.5)
     times = O.times_from_sigma(sigma, flow)
     hp = O.Hyper(n_steps=n, min_step_frac=1.0, flow=flow)
-    sampling = O.FlowSampling() if flow else O.VESampling()
     tape = O.NoiseTape(generator=torch.Generator().manual_seed(4))
-    want_out, want_x = O.outer_step(O.PointwiseDenoiser(sampling), x.clone(), y, noise, sigma, mask, times, hp,
-                                    n_steps=n, draw=tape)
-    replay = iter(tape.recorded)
+    sampling = O.FlowSampling() if flow else O.VESampling()
+    want = O.outer_step(O.PointwiseDenoiser(sampling), x.clone(), y, noise, sigma, mask, times, hp, n_steps=n, draw=tape)
+    return (x, y, noise, sigma, mask, times, hp), want, tape.recorded
+
+
+def run_reference(Ref, flow, n, args, draws, monkeypatch):
+    """The reference engine class `Ref` on one case, its torch.randn_like replaying `draws` -> (out, x)."""
+    x, y, noise, sigma, mask, times, hp = args
+    replay = iter(draws)
     monkeypatch.setattr(torch, "randn_like", lambda t, **kw: next(replay).to(t.dtype))
+    sampling = O.FlowSampling() if flow else O.VESampling()
     eng = Ref(O.PointwiseDenoiser(sampling), n, 15.0, hp.lam, hp.beta, hp.step_size, IS_FLUX=False, IS_FLOW=flow,
               MinStepFrac=1.0)
     xr = x.clone()
     out = eng(xr, y, noise, sigma, mask, tuple(times), {}, 0, n_steps=n)
+    return out, xr
+
+
+@pytest.mark.parametrize("flow,n,batch", CASES)
+def test_reference_bytecode_equals_the_port(flow, n, batch, monkeypatch):
+    args, (want_out, want_x), draws = port_case(flow, n, batch)
+    z = np.load(os.path.join(GOLDEN_DIR, "aux_ref_port_cases.npz"))
+    key = f"{int(flow)}_{n}_{batch}"
+    assert torch.equal(torch.from_numpy(z[key + "_out"]), want_out) and torch.equal(torch.from_numpy(z[key + "_x"]), want_x)
+    Ref = build_ref.load()
+    if Ref is None:
+        return          # the stored outputs above are the reference's; the live comparison needs oracle/_ref
+    out, xr = run_reference(Ref, flow, n, args, draws, monkeypatch)
     assert torch.equal(out, want_out) and torch.equal(xr, want_x)
 
 
