@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LP_ABI_VERSION 5
+#define LP_ABI_VERSION 6
 #define LP_TABLE_STRIDE 32 /* floats per table row (one 128-byte line), layout below */
 
 typedef void* lp_stream_t; /* a cudaStream_t / CUstream */
@@ -136,17 +136,11 @@ typedef struct lp_heads {
 int lp_abi_version(void);
 const char* lp_status_string(int status);
 int lp_last_cuda_error(void); /* cudaError_t of the last failed launch on this thread */
-/* Process-wide switches (also read once from the environment: LANPAINT_B200_PDL, LANPAINT_B200_TMA,
- * LANPAINT_B200_TMA_MIN, LANPAINT_B200_TMA_BOUNDARY):
+/* Process-wide switches (also read once from the environment: LANPAINT_B200_PDL, LANPAINT_B200_TMA):
  *   "pdl" 1|0      programmatic dependent launch on every kernel (default 1)
  *   "tma" 1|0      use the TMA-staged persistent variants (cp.async.bulk + mbarrier ring) of the fused sub-step
- *                  (philox and torch streams) and of the step-boundary kernel when eligible: spatial a multiple
- *                  of 16, no side outputs, no row split (default 1; 2..5 select alternative tile geometries of
- *                  the philox kernel and 8 the two-subsequences-per-thread geometry of the torch kernel, for
- *                  measurement)
- *   "tma_min"      smallest launch, in elements, that takes a TMA-staged variant (default 2^18)
- *   "tma_boundary" 1|0  lp_boundary: TMA-staged kernel when eligible | always the LDG kernel (default 0: measured
- *                  faster inside a job, where the network's output is still in L2) */
+ *                  (philox and torch streams) when eligible: at least 2^18 elements, spatial a multiple of 16,
+ *                  no side outputs, no row split (default 1) */
 int lp_set_option(const char* name, int value);
 
 /* Host-only self test of the index arithmetic the kernels rely on (the multiply-shift division that
@@ -321,20 +315,6 @@ int lp_synth_denoiser_f32(const float* x, float* h0, float* h1, int64_t n, const
 /* Same, heads written in `dtype` (a network that computes in bf16 returns bf16 predictions). */
 int lp_synth_denoiser(const float* x, void* h0, void* h1, int dtype, int64_t n, const float* coef5_host,
                       lp_stream_t stream);
-
-/* L2 residency for the operands every sub-step re-reads (the clean latent y and the mask: 4 + 1/C of the
- * 28 + 1/C bytes per element).  B200 has 126 MB of L2; pinning y (and the mask that follows it in the same
- * allocation, if any) with a persisting access-policy window turns those reads into L2 hits for the whole
- * job.  lp_l2_persist_set() raises cudaLimitPersistingL2CacheSize to cover `bytes` (clamped to the device
- * maximum; hit_ratio is scaled down accordingly) and installs the window on `stream`: every kernel launched
- * (or captured) on that stream afterwards carries it.  lp_l2_persist_clear() removes the window and resets the
- * persisting lines.  Both are host-side configuration calls, not captured operations. */
-int lp_l2_persist_capacity(int device, size_t* max_persisting_bytes, size_t* max_window_bytes);
-int lp_l2_persist_set(const void* ptr, size_t bytes, lp_stream_t stream);
-int lp_l2_persist_clear(lp_stream_t stream);
-
-/* Writes `bytes` of scratch (> L2) to evict the working set between launches. */
-int lp_l2_flush(void* scratch, size_t bytes, lp_stream_t stream);
 
 #ifdef __cplusplus
 }

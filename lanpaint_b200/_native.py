@@ -12,7 +12,7 @@ from typing import Optional
 _LIB_PATH = os.environ.get("LANPAINT_B200_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib",
                                                                "liblanpaint_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 TABLE_STRIDE = 32
 
 RNG_TAPE, RNG_PHILOX, RNG_TORCH = 0, 1, 2
@@ -25,7 +25,7 @@ SYMBOLS = (
     "lp_abi_version", "lp_status_string", "lp_last_cuda_error", "lp_set_option", "lp_selftest_index_math", "lp_selftest_box_muller", "lp_build_coef_table", "lp_build_coef_table_dt",
     "lp_torch_randn_geometry", "lp_pack_mask_f32", "lp_prologue_f32", "lp_substep", "lp_substep_f32", "lp_substep_cfg_f32", "lp_advance_f32",
     "lp_boundary", "lp_synth_denoiser",
-    "lp_epilogue_f32", "lp_epilogue_euler_f32", "lp_step_boundary_f32", "lp_epilogue_cfg_f32", "lp_stop_stats_f32", "lp_fill_normal_f32", "lp_synth_denoiser_f32", "lp_l2_persist_capacity", "lp_l2_persist_set", "lp_l2_persist_clear", "lp_l2_flush", "lp_torch_cpu_randn_f32",
+    "lp_epilogue_f32", "lp_epilogue_euler_f32", "lp_step_boundary_f32", "lp_epilogue_cfg_f32", "lp_stop_stats_f32", "lp_fill_normal_f32", "lp_synth_denoiser_f32", "lp_torch_cpu_randn_f32",
 )
 
 
@@ -121,14 +121,6 @@ def load() -> C.CDLL:
     lib.lp_fill_normal_f32.argtypes = [p, i64, C.POINTER(Rng), p]
     lib.lp_synth_denoiser_f32.restype = i32
     lib.lp_synth_denoiser_f32.argtypes = [p, p, p, i64, p, p]
-    lib.lp_l2_persist_capacity.restype = i32
-    lib.lp_l2_persist_capacity.argtypes = [i32, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
-    lib.lp_l2_persist_set.restype = i32
-    lib.lp_l2_persist_set.argtypes = [p, C.c_size_t, p]
-    lib.lp_l2_persist_clear.restype = i32
-    lib.lp_l2_persist_clear.argtypes = [p]
-    lib.lp_l2_flush.restype = i32
-    lib.lp_l2_flush.argtypes = [p, C.c_size_t, p]
     lib.lp_torch_cpu_randn_f32.restype = i32
     lib.lp_torch_cpu_randn_f32.argtypes = [p, i64, u64, p, C.POINTER(i64), p]
     v = lib.lp_abi_version()

@@ -1,7 +1,7 @@
 // lanpaint_b200: everything of an outer step that is not the fused sub-step.
 //   prologue_kernel     replace step + change of variables              lanpaint.py:85-99
 //   boundary_kernel     final paste [+ CFG combine] [+ k-diffusion Euler update] [+ next replace step]
-//                       lanpaint.py:151-157, sample_euler, lanpaint.py:85-94     (LDG and TMA-staged variants)
+//                       lanpaint.py:151-157, sample_euler, lanpaint.py:85-94
 //   advance_kernel      one un-fused advance_time_overdamped             lanpaint.py:232-254
 //   stop_stats_kernel   early-stop masked reductions                     earlystop.py:32-55,238-313
 #include "lp_common.cuh"
@@ -99,131 +99,8 @@ __global__ void __launch_bounds__(kBlock) boundary_kernel(const BoundaryArgs p) 
   if (euler) store_f<N>(p.x, i, xv);
 }
 
-// TMA-staged persistent variant for HBM-bound sizes (fused Euler loop: x is always updated).  Same tile walk and
-// mbarrier ring as substep_tma_kernel; kCombine / kNext select which slices a tile needs.
-template <typename H, int kTile>
-struct __align__(128) BoundaryStage {
-  H a[kTile], b[kTile];
-  float y[kTile], nz[kTile], x[kTile];
-  uint8_t m[kTile];
-};
-
-struct BTileGeom {
-  uint32_t tiles_per_channel, n_tiles, channels;
-};
-
-template <typename H, bool kCombine, bool kNext, int kTile, int kStages>
-__global__ void __launch_bounds__(kBlock, 2) boundary_tma_kernel(const BoundaryArgs p, const BTileGeom tg) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  using Stage = BoundaryStage<H, kTile>;
-  Stage* stage = reinterpret_cast<Stage*>(smem_raw);
-  __shared__ __align__(8) uint64_t full[kStages];
-  pdl_prologue();
-  const uint32_t S = p.g.spatial.d;
-  const H* ap = static_cast<const H*>(p.a);
-  const H* bp = static_cast<const H*>(p.b);
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int s = 0; s < kStages; ++s) mbar_init(&full[s], 1);
-    mbar_fence_init();
-  }
-  __syncthreads();
-  auto tile_origin = [&](uint32_t tile, uint32_t& e0, uint32_t& len, uint32_t& row, uint32_t& mi0) {
-    const uint32_t rc = tile / tg.tiles_per_channel;
-    const uint32_t s0 = (tile - rc * tg.tiles_per_channel) * kTile;
-    len = S - s0 < (uint32_t)kTile ? S - s0 : (uint32_t)kTile;
-    e0 = rc * S + s0;
-    row = rc / tg.channels;
-    mi0 = row * p.g.mask_row_stride + (rc - row * tg.channels) * p.g.mask_channel_stride + s0;
-  };
-  auto issue = [&](uint32_t tile, int s) {
-    uint32_t e0, len, row, mi0;
-    tile_origin(tile, e0, len, row, mi0);
-    const uint32_t fb = len * 4u, hb = len * (uint32_t)sizeof(H);
-    mbar_expect_tx(&full[s], fb * (2u + (kNext ? 1u : 0u)) + hb * (1u + (kCombine ? 1u : 0u)) + len);
-    Stage& t = stage[s];
-    tma_load_1d(t.a, ap + e0, hb, &full[s]);
-    if (kCombine) tma_load_1d(t.b, bp + e0, hb, &full[s]);
-    tma_load_1d(t.y, p.y + e0, fb, &full[s]);
-    if (kNext) tma_load_1d(t.nz, p.noise + e0, fb, &full[s]);
-    tma_load_1d(t.x, p.x + e0, fb, &full[s]);
-    tma_load_1d(t.m, p.mask + mi0, len, &full[s]);
-  };
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int s = 0; s < kStages; ++s) {
-      const uint32_t tile = blockIdx.x + (uint32_t)s * gridDim.x;
-      if (tile < tg.n_tiles) issue(tile, s);
-    }
-  }
-  uint32_t k = 0;
-  for (uint32_t tile = blockIdx.x; tile < tg.n_tiles; tile += gridDim.x, ++k) {
-    const int s = (int)(k % kStages);
-    mbar_wait(&full[s], (k / kStages) & 1u);
-    uint32_t e0, len, row, mi0;
-    tile_origin(tile, e0, len, row, mi0);
-    const Stage& t = stage[s];
-    float rn = 0.f, ry = 0.f;
-    if (kNext) {
-      rn = __ldg(p.next_table + (size_t)row * LP_TABLE_STRIDE + LP_T_REPN);
-      ry = __ldg(p.next_table + (size_t)row * LP_TABLE_STRIDE + LP_T_REPY);
-    }
-#pragma unroll
-    for (int pass = 0; pass < kTile / (4 * kBlock); ++pass) {
-      const uint32_t v = threadIdx.x + pass * kBlock;
-      if (4 * v < len) {
-        float av[4], bv[4] = {0.f, 0.f, 0.f, 0.f};
-        lds_head4<H>(t.a, v, av);
-        if (kCombine) lds_head4<H>(t.b, v, bv);
-        const float4 yv = reinterpret_cast<const float4*>(t.y)[v];
-        const float4 nv = kNext ? reinterpret_cast<const float4*>(t.nz)[v] : make_float4(0.f, 0.f, 0.f, 0.f);
-        const float4 xq = reinterpret_cast<const float4*>(t.x)[v];
-        const uchar4 mv = reinterpret_cast<const uchar4*>(t.m)[v];
-        float x[4] = {xq.x, xq.y, xq.z, xq.w}, o[4];
-        const float y[4] = {yv.x, yv.y, yv.z, yv.w}, nz[4] = {nv.x, nv.y, nv.z, nv.w};
-        const bool known[4] = {mv.x != 0, mv.y != 0, mv.z != 0, mv.w != 0};
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-          boundary_element(av[j], bv[j], y[j], nz[j], known[j], x[j], o[j], kCombine, p.cfg, p.coef, true, kNext, rn, ry);
-        const uint32_t i = e0 + 4 * v;
-        if (p.out) *reinterpret_cast<float4*>(p.out + i) = make_float4(o[0], o[1], o[2], o[3]);
-        *reinterpret_cast<float4*>(p.x + i) = make_float4(x[0], x[1], x[2], x[3]);
-      }
-    }
-    __syncthreads();
-    const uint32_t next = tile + (uint32_t)kStages * gridDim.x;
-    if (threadIdx.x == 0 && next < tg.n_tiles) issue(next, s);
-  }
-}
-
-template <typename H, bool kCombine, bool kNext>
-int launch_boundary_tma(const BoundaryArgs& p, cudaStream_t s) {
-  constexpr int kTile = 2048, kStages = 2;
-  const int dev = current_device();
-  const size_t smem = sizeof(BoundaryStage<H, kTile>) * kStages;
-  static bool configured[kMaxDevices] = {};  // per instantiation of this launcher
-  ensure_dynamic_smem(boundary_tma_kernel<H, kCombine, kNext, kTile, kStages>, smem, dev, configured);
-  BTileGeom tg;
-  tg.channels = p.g.per_row.d / p.g.spatial.d;
-  tg.tiles_per_channel = (p.g.spatial.d + kTile - 1) / kTile;
-  tg.n_tiles = (p.g.total / p.g.spatial.d) * tg.tiles_per_channel;
-  unsigned grid = (unsigned)device_info(dev).sms * 2u;
-  if (grid > tg.n_tiles) grid = tg.n_tiles;
-  launch_kernel_smem(boundary_tma_kernel<H, kCombine, kNext, kTile, kStages>, dim3(grid), smem, s, p, tg);
-  return check_launch();
-}
-
 template <typename H>
-int boundary_dispatch(const BoundaryArgs& p, bool v4, int dtype, cudaStream_t s) {
-  const bool tma = v4 && g_opt_tma != 0 && g_opt_tma_boundary != 0 && p.x && geometry_tma(p.g, p.mask) && p.g.total >= (uint32_t)g_opt_tma_min &&
-                   aligned16(p.a) && (!p.combine || aligned16(p.b)) && aligned16(p.y) && aligned16(p.x) &&
-                   (!p.next_table || aligned16(p.noise)) && (!p.out || aligned16(p.out));
-  if (tma) {
-    if (p.combine && p.next_table) return launch_boundary_tma<H, true, true>(p, s);
-    if (p.combine) return launch_boundary_tma<H, true, false>(p, s);
-    if (p.next_table) return launch_boundary_tma<H, false, true>(p, s);
-    return launch_boundary_tma<H, false, false>(p, s);
-  }
+int boundary_dispatch(const BoundaryArgs& p, bool v4, cudaStream_t s) {
   if (v4) launch_kernel(boundary_kernel<4, H>, dim3(blocks_for(p.g.total / 4)), s, p);
   else launch_kernel(boundary_kernel<1, H>, dim3(blocks_for(p.g.total)), s, p);
   return check_launch();
@@ -248,9 +125,9 @@ static int boundary_impl(const lp_heads* mo, const float* y, const float* noise,
                   (!out || aligned16(out));
   cudaStream_t s = (cudaStream_t)stream;
   switch (dtype) {
-    case LP_DTYPE_F32: return boundary_dispatch<float>(p, v4, dtype, s);
-    case LP_DTYPE_BF16: return boundary_dispatch<__nv_bfloat16>(p, v4, dtype, s);
-    default: return boundary_dispatch<__half>(p, v4, dtype, s);
+    case LP_DTYPE_F32: return boundary_dispatch<float>(p, v4, s);
+    case LP_DTYPE_BF16: return boundary_dispatch<__nv_bfloat16>(p, v4, s);
+    default: return boundary_dispatch<__half>(p, v4, s);
   }
 }
 

@@ -14,18 +14,6 @@ int g_opt_tma = [] {
   const char* e = getenv("LANPAINT_B200_TMA");
   return e ? atoi(e) : 1;
 }();
-int g_opt_tma_min = [] {
-  const char* e = getenv("LANPAINT_B200_TMA_MIN");
-  return e ? atoi(e) : (1 << 18);
-}();
-
-// Measured (profiles/README.md, round 2): inside a job the LDG boundary kernel beats the TMA-staged one (its inputs
-// were just written by the network and sit in L2, and it skips the operands a vector's mask makes unnecessary):
-// 4.17 vs 4.30 ms per 128-request job.  The TMA variant stays available, off by default.
-int g_opt_tma_boundary = [] {
-  const char* e = getenv("LANPAINT_B200_TMA_BOUNDARY");
-  return e ? atoi(e) : 0;
-}();
 
 int current_device() {
   int dev = 0;
@@ -228,8 +216,6 @@ extern "C" int lp_set_option(const char* name, int value) {
   const auto eq = [&](const char* k) { int i = 0; while (k[i] && name[i] == k[i]) ++i; return !k[i] && !name[i]; };
   if (eq("pdl")) { g_opt_pdl = value; return LP_OK; }
   if (eq("tma")) { g_opt_tma = value; return LP_OK; }
-  if (eq("tma_min")) { g_opt_tma_min = value; return LP_OK; }
-  if (eq("tma_boundary")) { g_opt_tma_boundary = value; return LP_OK; }
   return LP_ERR_INVALID;
 }
 
@@ -321,55 +307,4 @@ extern "C" int lp_synth_denoiser(const float* x, void* h0, void* h1, int dtype, 
 extern "C" int lp_synth_denoiser_f32(const float* x, float* h0, float* h1, int64_t n, const float* coef,
                                      lp_stream_t stream) {
   return lp_synth_denoiser(x, h0, h1, LP_DTYPE_F32, n, coef, stream);
-}
-
-extern "C" int lp_l2_persist_capacity(int device, size_t* max_persisting_bytes, size_t* max_window_bytes) {
-  if (device < 0 && cudaGetDevice(&device) != cudaSuccess) return LP_ERR_CUDA;
-  int a = 0, b = 0;
-  if (cudaDeviceGetAttribute(&a, cudaDevAttrMaxPersistingL2CacheSize, device) != cudaSuccess ||
-      cudaDeviceGetAttribute(&b, cudaDevAttrMaxAccessPolicyWindowSize, device) != cudaSuccess) {
-    g_last_cuda_error = static_cast<int>(cudaGetLastError());
-    return LP_ERR_CUDA;
-  }
-  if (max_persisting_bytes) *max_persisting_bytes = (size_t)a;
-  if (max_window_bytes) *max_window_bytes = (size_t)b;
-  return LP_OK;
-}
-
-extern "C" int lp_l2_persist_set(const void* ptr, size_t bytes, lp_stream_t stream) {
-  if (!ptr || bytes == 0) return LP_ERR_INVALID;
-  size_t cap = 0, win = 0;
-  if (int rc = lp_l2_persist_capacity(-1, &cap, &win)) return rc;
-  if (cap == 0 || win == 0) return LP_ERR_UNSUPPORTED;
-  const size_t want = bytes < cap ? bytes : cap;
-  if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) != cudaSuccess) return (check_launch(), LP_ERR_CUDA);
-  cudaStreamAttrValue v;
-  v.accessPolicyWindow.base_ptr = const_cast<void*>(ptr);
-  v.accessPolicyWindow.num_bytes = bytes < win ? bytes : win;
-  v.accessPolicyWindow.hitRatio = (float)((double)want / (double)(bytes < win ? bytes : win));
-  if (v.accessPolicyWindow.hitRatio > 1.f) v.accessPolicyWindow.hitRatio = 1.f;
-  v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-  v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  if (cudaStreamSetAttribute((cudaStream_t)stream, cudaStreamAttributeAccessPolicyWindow, &v) != cudaSuccess)
-    return (check_launch(), LP_ERR_CUDA);
-  return LP_OK;
-}
-
-extern "C" int lp_l2_persist_clear(lp_stream_t stream) {
-  cudaStreamAttrValue v;
-  v.accessPolicyWindow.base_ptr = nullptr;
-  v.accessPolicyWindow.num_bytes = 0;
-  v.accessPolicyWindow.hitRatio = 0.f;
-  v.accessPolicyWindow.hitProp = cudaAccessPropertyNormal;
-  v.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-  cudaStreamSetAttribute((cudaStream_t)stream, cudaStreamAttributeAccessPolicyWindow, &v);
-  if (cudaCtxResetPersistingL2Cache() != cudaSuccess) return (check_launch(), LP_ERR_CUDA);
-  cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0);  // give the set-aside back to normal traffic
-  return LP_OK;
-}
-
-extern "C" int lp_l2_flush(void* scratch, size_t bytes, lp_stream_t stream) {
-  if (!scratch) return LP_ERR_INVALID;
-  if (cudaMemsetAsync(scratch, 0, bytes, (cudaStream_t)stream) != cudaSuccess) return (check_launch(), LP_ERR_CUDA);
-  return LP_OK;
 }

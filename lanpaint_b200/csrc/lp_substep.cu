@@ -453,171 +453,9 @@ __device__ __forceinline__ void torch_tma_body(const SubstepArgs& a, const Torch
   }
 }
 
-// ---- the same kernel with TWO subsequences per consumer thread ---------------------------------------------------
-// Half the per-thread state (2 Philox calls per draw, one FP32x2 Box-Muller call per draw and half, one FP32x2 update
-// per plane, LDS.64 / STG.64), so the register ceiling can drop to 64 and twice as many consumer warps fit per SM:
-// the kernel is bound by issue latency, not by the pipes.  Groups of kG subsequences need not divide T.
-template <typename H, bool kFirst, bool kNext, int kG>
-__device__ __forceinline__ void torch_tma_body2(const SubstepArgs& a, const TorchTmaGeom& tg, unsigned char* smem_raw,
-                                                uint64_t* full, uint64_t* empty) {
-  constexpr int kConsumers = kG / 2;
-  using Slot = TorchSlot<H, kG>;
-  Slot* slot = reinterpret_cast<Slot*>(smem_raw);
-  pdl_prologue();
-  const uint32_t T = a.torch_T, total = a.g.total;
-  const bool aliased = a.x0b == a.x0;
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      mbar_init(&full[j], 1);
-      mbar_init(&empty[j], kConsumers);
-    }
-    mbar_fence_init();
-  }
-  __syncthreads();
-  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-  // first element / length of sub-tile j of group (k, b): clipped by the end of the plane and of the tensor
-  auto subtile = [&](uint32_t k, uint32_t b, int j, uint32_t& e0, uint32_t& len) {
-    const uint32_t in_plane = T - b * kG < (uint32_t)kG ? T - b * kG : (uint32_t)kG;
-    const uint64_t e = (uint64_t)(4u * k + (uint32_t)j) * T + (uint64_t)b * kG;
-    if (e >= total) {
-      e0 = 0;
-      len = 0;
-    } else {
-      e0 = (uint32_t)e;
-      len = total - e0 < in_plane ? total - e0 : in_plane;
-    }
-  };
-
-  if (warp == kConsumers / 32) {  // ---------------- producer ----------------
-    if (lane == 0) {
-      const H* x0p = static_cast<const H*>(a.x0);
-      const H* x0bp = static_cast<const H*>(a.x0b);
-      uint32_t it = 0;
-      for (uint32_t grp = blockIdx.x; grp < tg.n_groups; grp += gridDim.x, ++it) {
-        const uint32_t k = grp / tg.groups_per_call, b = grp - k * tg.groups_per_call;
-#pragma unroll 1
-        for (int j = 0; j < 4; ++j) {
-          mbar_wait_relaxed(&empty[j], (it & 1u) ^ 1u);
-          uint32_t e0, len;
-          subtile(k, b, j, e0, len);
-          const uint32_t fb = len * 4u, hb = len * (uint32_t)sizeof(H);
-          mbar_expect_tx(&full[j], fb * (2u + (kFirst ? 0u : 1u)) + hb * (1u + (aliased ? 0u : 1u)) + len);
-          if (len == 0) continue;
-          Slot& t = slot[j];
-          tma_load_1d(t.x, a.x + e0, fb, &full[j]);
-          tma_load_1d(t.x0, x0p + e0, hb, &full[j]);
-          if (!aliased) tma_load_1d(t.x0b, x0bp + e0, hb, &full[j]);
-          tma_load_1d(t.y, a.y + e0, fb, &full[j]);
-          if (!kFirst) tma_load_1d(t.c, a.c + e0, fb, &full[j]);
-          uint32_t e = e0, off = 0, rem = len;
-          while (rem) {
-            const uint32_t row = a.g.per_row.div(e);
-            const uint32_t r = e - row * a.g.per_row.d;
-            const uint32_t ch = a.g.spatial.div(r);
-            const uint32_t s = r - ch * a.g.spatial.d;
-            const uint32_t seg = rem < a.g.spatial.d - s ? rem : a.g.spatial.d - s;
-            tma_load_1d(t.m + off, a.mask + row * a.g.mask_row_stride + ch * a.g.mask_channel_stride + s, seg,
-                        &full[j]);
-            e += seg;
-            off += seg;
-            rem -= seg;
-          }
-        }
-      }
-    }
-    return;
-  }
-
-  // ---------------- consumers ----------------
-  uint64_t seed = a.seed, o0 = a.draw0, o1 = a.draw1;
-  if (a.rng_state) {
-    seed = a.rng_state[0];
-    o0 += a.rng_state[1];
-    o1 += a.rng_state[1];
-  }
-  const uint32_t tid = threadIdx.x;  // pair index inside every sub-tile
-  uint32_t it = 0;
-  for (uint32_t grp = blockIdx.x; grp < tg.n_groups; grp += gridDim.x, ++it) {
-    const uint32_t k = grp / tg.groups_per_call, b = grp - k * tg.groups_per_call;
-    const uint32_t t0 = b * kG + 2u * tid;  // my two Philox subsequences (torch threads)
-    const uint4 ra0 = torch_philox(seed, o0, t0, k), ra1 = torch_philox(seed, o0, t0 + 1u, k);
-    uint4 rb0 = make_uint4(0u, 0u, 0u, 0u), rb1 = rb0;
-    if (kNext) {
-      rb0 = torch_philox(seed, o1, t0, k);
-      rb1 = torch_philox(seed, o1, t0 + 1u, k);
-    }
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {  // curand_normal4: planes 0,1 <- (x,y), planes 2,3 <- (z,w)
-      float2 p1[2], p2[2];
-      box_muller_curand_x2(h ? ra0.z : ra0.x, h ? ra0.w : ra0.y, h ? ra1.z : ra1.x, h ? ra1.w : ra1.y, p1[0], p1[1]);
-      if (kNext) {
-        box_muller_curand_x2(h ? rb0.z : rb0.x, h ? rb0.w : rb0.y, h ? rb1.z : rb1.x, h ? rb1.w : rb1.y, p2[0], p2[1]);
-      } else {
-        p2[0] = p2[1] = make_float2(0.f, 0.f);
-      }
-#pragma unroll
-      for (int jj = 0; jj < 2; ++jj) {
-        const int j = 2 * h + jj;
-        uint32_t e0, len;
-        subtile(k, b, j, e0, len);
-        mbar_wait(&full[j], it & 1u);
-        const bool active = 2u * tid < len;
-        float x[2] = {0.f, 0.f}, x0[2] = {0.f, 0.f}, x0b[2] = {0.f, 0.f}, y[2] = {0.f, 0.f}, cp[2] = {0.f, 0.f};
-        uchar2 mv = make_uchar2(0, 0);
-        if (active) {
-          const Slot& t = slot[j];
-          const float2 xv = reinterpret_cast<const float2*>(t.x)[tid];
-          lds_head2<H>(t.x0, tid, x0);
-          if (aliased) {
-            x0b[0] = x0[0];
-            x0b[1] = x0[1];
-          } else {
-            lds_head2<H>(t.x0b, tid, x0b);
-          }
-          const float2 yv = reinterpret_cast<const float2*>(t.y)[tid];
-          const float2 cv = kFirst ? make_float2(0.f, 0.f) : reinterpret_cast<const float2*>(t.c)[tid];
-          mv = reinterpret_cast<const uchar2*>(t.m)[tid];
-          x[0] = xv.x; x[1] = xv.y;
-          y[0] = yv.x; y[1] = yv.y;
-          cp[0] = cv.x; cp[1] = cv.y;
-        }
-        mbar_arrive(&empty[j]);  // my reads of slot j are in registers
-        if (active) {
-          const uint32_t i = e0 + 2u * tid;
-          const uint32_t row = a.g.per_row.div(i);
-          RowCoef<kFirst, kNext> rc;
-          rc.load(a.table + (size_t)row * LP_TABLE_STRIDE);
-          if (a.use_cfg) {
-            cfg_combine(x0[0], x0b[0], a.cfg, a.cfg_big);
-            cfg_combine(x0[1], x0b[1], a.cfg, a.cfg_big);
-          }
-          const bool known[2] = {mv.x != 0, mv.y != 0};
-          const float n1[2] = {jj ? p1[0].y : p1[0].x, jj ? p1[1].y : p1[1].x};
-          const float n2[2] = {jj ? p2[0].y : p2[0].x, jj ? p2[1].y : p2[1].x};
-          float cn[2];
-          substep_element_x2<kFirst, kNext>(x, x0, x0b, y, cp, known, n1, n2, rc, cn);
-          *reinterpret_cast<float2*>(a.x + i) = make_float2(x[0], x[1]);
-          if (kNext || a.store_c) *reinterpret_cast<float2*>(a.c + i) = make_float2(cn[0], cn[1]);
-        }
-      }
-    }
-  }
-}
-
-// <448 subsequences per group, 224 consumer threads + producer warp = 256 threads, up to 4 CTAs per SM, 64 registers>.
-// Bit-identical to the default geometry and measured SLOWER (48.7 vs 43.6 us per launch at R=128; with 3 CTAs per SM
-// and 80 registers 50.3 us): kept selectable (lp_set_option("tma", 8)) as the reproducible form of that result.
-template <typename H, bool kFirst, bool kNext>
-__global__ void __launch_bounds__(448 / 2 + 32, 4) substep_torch_tma_kernel_p2(const SubstepArgs a, const TorchTmaGeom tg) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  __shared__ __align__(8) uint64_t full[4], empty[4];
-  torch_tma_body2<H, kFirst, kNext, 448>(a, tg, smem_raw, full, empty);
-}
-// The default geometry: <1024 subsequences per group, 256 consumer threads + producer warp, 2 CTAs per SM, 96
-// registers>.  Measured and dropped: a 112-register ceiling (one CTA per SM, 70 us) and 2048-subsequence groups with 17
-// warps (does not launch).
+// <1024 subsequences per group, 256 consumer threads + producer warp, 2 CTAs per SM, 96 registers>.  Measured and
+// dropped: a 112-register ceiling (one CTA per SM, 70 us), 2048-subsequence groups with 17 warps (does not launch) and
+// two subsequences per thread in groups of 448 (48.7 vs 43.6 us per launch at R=128).
 template <typename H, bool kFirst, bool kNext>
 __global__ void __launch_bounds__(1024 / 4 + 32, 2) substep_torch_tma_kernel(const SubstepArgs a, const TorchTmaGeom tg) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -726,8 +564,11 @@ __global__ void __launch_bounds__(kBlock) substep_torch_kernel(const SubstepArgs
 // ----------------------------------------------------------------------------
 // launchers
 // ----------------------------------------------------------------------------
-template <typename H, bool kFirst, bool kNext, bool kMerge, int kTile, int kStages, int kMinBlocks>
-int launch_substep_tma_cfg(const SubstepArgs& a, cudaStream_t s) {
+// 2048-element tiles, 2 stages, 2 CTAs per SM: the fastest of the (tile, stages, CTAs per SM) geometries measured on the
+// steady fp32 kernel; 1024x4x2, 4096x2x1, 2048x4x1 and 1024x3x3 lost
+template <typename H, bool kFirst, bool kNext, bool kMerge>
+int launch_substep_tma(const SubstepArgs& a, cudaStream_t s) {
+  constexpr int kTile = 2048, kStages = 2, kMinBlocks = 2;
   const int dev = current_device();
   const size_t smem = sizeof(TmaStage<H, kTile>) * kStages;
   static bool configured[kMaxDevices] = {};  // per instantiation of this launcher
@@ -742,26 +583,10 @@ int launch_substep_tma_cfg(const SubstepArgs& a, cudaStream_t s) {
   return check_launch();
 }
 
-// tile / ring geometry: "tma" option value 1 (default) = 2048-element tiles, 2 stages, 2 CTAs per SM;
-// 2..5 are the alternatives measured in profiles/README.md (fp32 heads, steady kernel only)
-template <typename H, bool kFirst, bool kNext, bool kMerge>
-int launch_substep_tma(const SubstepArgs& a, cudaStream_t s) {
-  if constexpr (kNext && !kFirst && kMerge && sizeof(H) == 4) {
-    switch (g_opt_tma) {
-      case 2: return launch_substep_tma_cfg<H, kFirst, kNext, kMerge, 1024, 4, 2>(a, s);
-      case 3: return launch_substep_tma_cfg<H, kFirst, kNext, kMerge, 4096, 2, 1>(a, s);
-      case 4: return launch_substep_tma_cfg<H, kFirst, kNext, kMerge, 2048, 4, 1>(a, s);
-      case 5: return launch_substep_tma_cfg<H, kFirst, kNext, kMerge, 1024, 3, 3>(a, s);
-      default: break;
-    }
-  }
-  return launch_substep_tma_cfg<H, kFirst, kNext, kMerge, 2048, 2, 2>(a, s);
-}
-
 // The TMA-staged variants need 16-byte aligned slices (spatial a multiple of 16), no side outputs, no row split;
 // only worth it when there are enough tiles to keep a persistent grid busy.
 inline bool tma_eligible(const SubstepArgs& a) {
-  return g_opt_tma != 0 && geometry_tma(a.g, a.mask) && !a.x_copy && !a.x0e && a.g.total >= (uint32_t)g_opt_tma_min &&
+  return g_opt_tma != 0 && geometry_tma(a.g, a.mask) && !a.x_copy && !a.x0e && a.g.total >= kTmaMinElements &&
          aligned16(a.x) && aligned16(a.x0) && aligned16(a.x0b) && aligned16(a.y) && (!a.c || aligned16(a.c));
 }
 
@@ -795,19 +620,6 @@ int launch_substep_vec(const SubstepArgs& a, bool first, bool next, bool merge, 
 template <typename H, bool kFirst, bool kNext>
 int launch_torch_tma(const SubstepArgs& a, uint32_t calls, cudaStream_t s) {
   const int dev = current_device();
-  const int variant = (sizeof(H) == 4 && !kFirst && kNext) ? g_opt_tma : 1;   // the alternative: steady fp32 kernel only
-  if (variant == 8) {   // two subsequences per thread, groups of 448 (need not divide T)
-    const size_t smem = sizeof(TorchSlot<H, 448>) * 4;
-    TorchTmaGeom tg;
-    tg.groups_per_call = (a.torch_T + 447u) / 448u;
-    tg.n_groups = calls * tg.groups_per_call;
-    unsigned grid = (unsigned)device_info(dev).sms * 4u;
-    if (grid > tg.n_groups) grid = tg.n_groups;
-    static bool configured[kMaxDevices] = {};
-    ensure_dynamic_smem(substep_torch_tma_kernel_p2<H, kFirst, kNext>, smem, dev, configured);
-    launch_kernel_ex(substep_torch_tma_kernel_p2<H, kFirst, kNext>, dim3(grid), dim3(448 / 2 + 32), smem, s, a, tg);
-    return check_launch();
-  }
   const size_t smem = sizeof(TorchSlot<H, 1024>) * 4;
   TorchTmaGeom tg;
   tg.groups_per_call = a.torch_T / 1024;

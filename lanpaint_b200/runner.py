@@ -252,16 +252,10 @@ class GraphedJob:
     per-sigma wrapper (asserted bit-for-bit by the tests)."""
 
     def __init__(self, engine, sched: HostSchedule, shape, device, flow: bool = False, fused_euler: bool = True,
-                 l2_persist: bool = False, model_options=None, seed=0, external_init: bool = False,
-                 first_replace_noop=None):
+                 model_options=None, seed=0, external_init: bool = False, first_replace_noop=None):
         import numpy as np
         from .engine import _DrawPlan
         self.fused_euler = fused_euler   # Euler update inside lp_epilogue_euler_f32 instead of two torch kernels
-        # optional persisting-L2 window over the clean latent (re-read by every launch).  Measured on B200 at
-        # R=128: 3.97 ms/job with the window vs 3.39 ms without (the 33 MB set-aside costs more write absorption
-        # than the y hits give back), so it is off by default; see profiles/README.md
-        self.l2_persist = l2_persist
-        self.l2_window = 0
         from .schedule import Hyper, build_table, mean_half_dt
         if engine.rng not in ("philox", "torch"):
             raise ValueError("GraphedJob needs an in-kernel RNG mode ('philox' or 'torch')")
@@ -372,18 +366,10 @@ class GraphedJob:
                 torch.cuda.current_stream(self.device).wait_stream(side)
                 eng.launches, eng.model_calls, eng.substeps_done = counts
             graph = torch.cuda.CUDAGraph()
-            lib = _native.load()
             cap_stream = torch.cuda.Stream(device=self.device)
-            cap = C.c_void_p(cap_stream.cuda_stream)
-            if self.l2_persist:   # configured before capture begins; the window then rides on every captured kernel node
-                nbytes = self.y.numel() * 4
-                if lib.lp_l2_persist_set(C.c_void_p(self.y.data_ptr()), nbytes, cap) == 0:
-                    self.l2_window = nbytes
             cap_stream.wait_stream(torch.cuda.current_stream(self.device))
             with torch.cuda.graph(graph, stream=cap_stream):
                 fn(plan)
-            if self.l2_window:
-                lib.lp_l2_persist_clear(cap)
         finally:
             eng.kernel_timer = timer
         stats = (eng.launches - counts[0], eng.model_calls - counts[1])

@@ -19,7 +19,7 @@ ap.add_argument("--requests", type=int, default=128)
 ap.add_argument("--rng", default="philox")
 ap.add_argument("--no-merge", action="store_true")
 ap.add_argument("--mask", default="random", choices=["random", "blob"])
-ap.add_argument("--tma", type=int, default=1, help="0 = LDG kernel, 1 = TMA-staged (default), 2-5 = alternative tile geometries")
+ap.add_argument("--tma", type=int, default=1, help="0 = LDG, 1 = TMA-staged (default)")
 ap.add_argument("--rotate", type=int, default=3, help="independent operand sets cycled (1 = L2-assisted)")
 args = ap.parse_args()
 dev = torch.device("cuda:0")

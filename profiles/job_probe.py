@@ -1,7 +1,7 @@
 """runner.GraphedJob (whole-job graph, device-resident inputs) at a given batch size: ms per job.
 
     python profiles/job_probe.py --requests 256 [--rng philox] [--net two_head|cond_uncond]
-Environment switches of the library (LANPAINT_B200_TMA, LANPAINT_B200_TMA_BOUNDARY, LANPAINT_B200_TMA_MIN) apply."""
+The library's LANPAINT_B200_TMA environment switch applies."""
 import argparse
 import os
 import sys

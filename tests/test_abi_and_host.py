@@ -27,7 +27,7 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
     assert sorted(_native.SYMBOLS) == declared, "binding list and header drifted apart"
-    assert lib.lp_abi_version() == _native.ABI_VERSION == 5
+    assert lib.lp_abi_version() == _native.ABI_VERSION == 6
 
 
 def test_struct_layouts_match_header():
@@ -166,7 +166,8 @@ def test_oversized_and_malformed_geometry_is_refused_before_any_launch():
     empty = _native.Dims(0, 64, 16, 64, 16, 0)                       # empty batch: a no-op that succeeds
     assert lib.lp_epilogue_f32(fake, fake, fake, fake, C.byref(empty), None) == 0
     assert lib.lp_substep_f32(fake, fake, fake, fake, fake, fake, None, None, fake, C.byref(empty), C.byref(r), 9, None) == 1
-    assert lib.lp_set_option(b"no-such-option", 1) == 1
+    for name in (b"no-such-option", b"tma_boundary", b"tma_min"):
+        assert lib.lp_set_option(name, 1) == 1, name
 
 
 def test_host_schedule_reproduces_the_reference_step_counts():

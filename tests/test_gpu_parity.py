@@ -744,17 +744,16 @@ def test_torch_stream_tma_variant_is_bit_identical(cuda_device):
             x, y, noise, m = synth_inputs(shape, seed=33, device=dev)
             sig = torch.full((shape[0],), 1.3)
             times = tuple(O.times_from_sigma(sig, False))
-            for tma in (0, 1, 8):     # LDG kernels, the default TMA geometry, two subsequences per thread
+            for tma in (0, 1):     # LDG kernels, TMA kernel
                 assert lib.lp_set_option(b"tma", tma) == 0
                 torch.manual_seed(23)
                 eng = _engine(SynthDenoiser(VESampling()), dict(n_steps=4), rng="torch", batched_replace="per_sample")
                 xx = x.clone()
                 out = eng(xx, y, noise, sig, m, times, None, 0, n_steps=4)
                 res[(shape, tma)] = (out, xx, torch.cuda.default_generators[dev.index or 0].get_offset())
-            for tma in (1, 8):
-                assert torch.equal(res[(shape, 0)][0], res[(shape, tma)][0]), (shape, tma)
-                assert torch.equal(res[(shape, 0)][1], res[(shape, tma)][1]), (shape, tma)
-                assert res[(shape, 0)][2] == res[(shape, tma)][2]
+            assert torch.equal(res[(shape, 0)][0], res[(shape, 1)][0]), shape
+            assert torch.equal(res[(shape, 0)][1], res[(shape, 1)][1]), shape
+            assert res[(shape, 0)][2] == res[(shape, 1)][2]
     finally:
         lib.lp_set_option(b"tma", 1)
 
@@ -800,14 +799,14 @@ def test_tma_variants_with_fused_cfg_combine(rng, cuda_device):
 
 @pytest.mark.parametrize("combine,with_next,with_out", [(False, True, False), (False, True, True), (True, True, True),
                                                          (False, False, True), (True, False, False)])
-def test_boundary_tma_variant_is_bit_identical(combine, with_next, with_out, cuda_device):
-    """lp_boundary: the cp.async.bulk variant of the step boundary (epilogue + Euler update + next replace step,
-    optional CFG combine) against the LDG kernel and against plain torch, through the C ABI."""
+def test_boundary_matches_torch(combine, with_next, with_out, cuda_device):
+    """lp_boundary: the step boundary (epilogue + Euler update + next replace step, optional CFG combine) against
+    plain torch, through the C ABI."""
     from lanpaint_b200 import _native
     from lanpaint_b200.schedule import Hyper, build_table
     lib = _native.load()
     dev = cuda_device
-    B, Cc, S = 6, 4, 128 * 128 + 32 * 16     # ragged last tile
+    B, Cc, S = 6, 4, 128 * 128 + 32 * 16
     shape = (B, Cc, S)
     gen = torch.Generator(device=dev).manual_seed(1)
     a, b, y, nz, x0 = (torch.randn(shape, device=dev, generator=gen) for _ in range(5))
@@ -820,23 +819,13 @@ def test_boundary_tma_variant_is_bit_identical(combine, with_next, with_out, cud
     P = C.c_void_p
     coef, cfg = -0.37, 3.5
 
-    def run(tma):
-        assert lib.lp_set_option(b"tma", tma) == 0 and lib.lp_set_option(b"tma_boundary", tma) == 0
-        x, out = x0.clone(), torch.full(shape, float("nan"), device=dev)
-        h = _native.Heads(a.data_ptr(), b.data_ptr() if combine else None, _native.DTYPE_F32, 1 if combine else 0, cfg, cfg)
-        rc = lib.lp_boundary(C.byref(h), P(y.data_ptr()), P(nz.data_ptr()) if with_next else None, P(m8.data_ptr()),
-                             P(x.data_ptr()), P(out.data_ptr()) if with_out else None, C.c_float(coef),
-                             P(tab.data_ptr()) if with_next else None, C.byref(dims),
-                             P(torch.cuda.current_stream().cuda_stream))
-        assert rc == 0
-        return x, out
-    try:
-        x1, o1 = run(1)
-        x0_, o0 = run(0)
-    finally:
-        lib.lp_set_option(b"tma", 1)
-        lib.lp_set_option(b"tma_boundary", 0)   # the default (the LDG kernel measured faster inside a job)
-    assert torch.equal(x1, x0_)
+    x1, o1 = x0.clone(), torch.full(shape, float("nan"), device=dev)
+    h = _native.Heads(a.data_ptr(), b.data_ptr() if combine else None, _native.DTYPE_F32, 1 if combine else 0, cfg, cfg)
+    rc = lib.lp_boundary(C.byref(h), P(y.data_ptr()), P(nz.data_ptr()) if with_next else None, P(m8.data_ptr()),
+                         P(x1.data_ptr()), P(o1.data_ptr()) if with_out else None, C.c_float(coef),
+                         P(tab.data_ptr()) if with_next else None, C.byref(dims),
+                         P(torch.cuda.current_stream().cuda_stream))
+    assert rc == 0
     known = m8.bool().expand(shape)
     d = b + (a - b) * cfg if combine else a
     o = torch.where(known, y, d)
@@ -847,7 +836,7 @@ def test_boundary_tma_variant_is_bit_identical(combine, with_next, with_out, cud
         xe = torch.where(known, rn * nz + ry * y, xe)
     assert (x1 - xe).abs().max().item() <= 1e-5 * max(1.0, xe.abs().max().item())
     if with_out:
-        assert torch.equal(o1, o0) and torch.equal(o1, o)
+        assert torch.equal(o1, o)
 
 
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
